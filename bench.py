@@ -13,10 +13,12 @@ The same JSON line also carries, inside parsed keys:
   e2e.stream_p50_ms         BASELINE configs[4]: p50 per-scan latency of a 10 Hz stream (~50 buckets / scan, 400 Hz
                             inertial queue, map updated after every bucket) through lk_process_scan with host buffers
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...    (one rank per GPU; scans shard, no collective on the hot path)
 
-Prints ONE JSON line (rank 0). Point-iteration = one point through one iteration.
+Prints ONE JSON line (rank 0). Point-iteration = one point through one iteration. --dump-outputs DIR writes what the
+timed path returned in its last step (state, covariance, clocks, success counts, world cloud) as DIR/<name>.npy; the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -27,6 +29,7 @@ import threading
 import time
 
 import numpy as np
+from numpy.lib import recfunctions
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "leg-kilo_b200", "python"))
@@ -52,6 +55,33 @@ WORKLOADS = {
                   baseline_config="smoke-size variant of configs[1]"),
 }
 LIDARS = dict(VLP16=synth.VLP16, OS64=synth.OS64, SYNTH100K=SYNTH100K)
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Writes d/<name>.npy for each array: float64, point clouds float32. A cloud that would take the files past
+    DUMP_BYTES is cut to a fixed, seeded sample of rows, whose indices go to d/<name>_rows.npy."""
+    os.makedirs(d, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.names:
+            a = recfunctions.structured_to_unstructured(a, dtype=np.float64)
+        out[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    clouds = [k for k, a in out.items() if a.dtype == np.float32]
+    room = DUMP_BYTES - sum(a.nbytes for k, a in out.items() if k not in clouds) - 256 * (len(out) + len(clouds))  # .npy headers
+    for k in clouds:
+        a = out[k]
+        if a.nbytes <= room // len(clouds):
+            continue
+        keep = max(room // len(clouds), 0) // (a.nbytes // len(a) + 8)  # a row and its float64 index
+        if len(a) > keep:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            out[k] = a[rows]
+            out[k + "_rows"] = rows.astype(np.float64)
+    for k, a in out.items():
+        np.save(os.path.join(d, k + ".npy"), a)
 
 
 def ncu_traffic_family():
@@ -320,7 +350,7 @@ def stream_run(cfgname, n_timed, n_warm, impl_ref, device=0, params=()):
             o.set_filter(x, P, Q, clk)
             r = o.process_scan(t0, pts, imu=None if kin_mode else meas, kin=meas if kin_mode else None)
             xo, Po, _, co = o.get_filter()
-            return xo, Po.reshape(1, 900), co, r["n_eff"]
+            return xo, Po.reshape(1, 900), co, r["n_eff"], r["world"]
     else:
         eng = Engine(cfg, device=device)
         for kv in params:
@@ -331,7 +361,7 @@ def stream_run(cfgname, n_timed, n_warm, impl_ref, device=0, params=()):
         def proc(x, P, clk, pts, offs, times, meas, t0):
             out = eng.process_scan(x, P, Q, clk, pts, offs, times, imu=None if kin_mode else meas, kin=meas if kin_mode else None,
                                    gravity=9.81, acc_norm=9.79, iters=1, update_map=True)
-            return out["x"], out["P"].reshape(1, 900), out["clk"], out["n_eff"]
+            return out["x"], out["P"].reshape(1, 900), out["clk"], out["n_eff"], out["world"]
     x = abi.default_states(1); P = abi.init_cov(1); clk = np.zeros(1, abi.CLOCK_DTYPE)
     lat, neff = [], []
     for i, sc in enumerate(scans):
@@ -340,19 +370,22 @@ def stream_run(cfgname, n_timed, n_warm, impl_ref, device=0, params=()):
         meas = (synth.kinimu_stream if kin_mode else synth.imu_stream)(t0 - 0.1 if i else -0.005, t0 + 0.1, 400.0, stream=9000 + i)
         meas = meas[meas["stamp"] > float(clk["last_update_time"][0]) - 1.0]
         a = time.perf_counter()
-        x, P, clk, ne = proc(x, P, clk, pts, offs, times, meas, t0)
+        x, P, clk, ne, world = proc(x, P, clk, pts, offs, times, meas, t0)
         lat.append(1e3 * (time.perf_counter() - a)); neff.append(ne)
     return dict(lat=np.array(lat[n_warm:]), neff=np.array(neff[n_warm:]), kin_mode=kin_mode,
-                points_per_scan=int(np.mean([len(s) for s in scans])))
+                points_per_scan=int(np.mean([len(s) for s in scans])),
+                last=dict(x=x, P=P.reshape(1, 30, 30), clk=clk, n_eff=np.array([ne]), world=world))
 
 
 def stream_latency(args):
     if int(os.environ.get("RANK", "0")) != 0:
         return 0
     cfgname = "nclt" if args.workload == "nclt_stream" else "leg_fusion"
-    K, W = max(args.steps, 8), max(args.warmup, 3)
+    K, W = args.steps, max(args.warmup, 3)
     impl_ref = args.impl == "reference"
     r = stream_run(cfgname, K, W, impl_ref, device=int(os.environ.get("LOCAL_RANK", "0")), params=args.param)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["last"])
     lat = r["lat"]
     line = dict(metric="p50 per-scan latency of the streaming ESKF LiDAR update (10 Hz, ~50 buckets/scan, map updated per bucket)",
                 value=float(np.median(lat)), unit="ms", n_gpus=1, steps=K, warmup=W, ms_per_step=float(np.mean(lat)),
@@ -439,8 +472,8 @@ def throughput_mode(args, rank, world, local_rank, dist, hbm_peak):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=4096)
-    ap.add_argument("--warmup", type=int, default=512)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 4096, streaming workloads 100)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 512, streaming workloads 5)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="leg_fusion_b1", choices=sorted(WORKLOADS) + ["nclt_stream", "leg_fusion_stream"])
     ap.add_argument("--scans", type=int, default=0, help="ring size (distinct scans staged in HBM)")
@@ -453,10 +486,16 @@ def main():
     ap.add_argument("--no-stream", action="store_true", help="skip e2e.stream_p50_ms (configs[4])")
     ap.add_argument("--param", action="append", default=[], help="engine parameter name=value (lk_set_param), repeatable")
     ap.add_argument("--fused", type=int, default=-1, help="0 = force the multi-kernel path for batch-of-one runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
-    if args.workload.endswith("_stream"):
-        if args.steps == 4096:
-            args.steps, args.warmup = 100, 5
+    stream = args.workload.endswith("_stream")
+    if args.steps is None:
+        args.steps = 100 if stream else 4096
+    if args.warmup is None:
+        args.warmup = 5 if stream else 512
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if stream:
         return stream_latency(args)
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -464,7 +503,7 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     ring = args.scans or w["ring"]
     ring = max(ring, w["batch"])
-    K, W = max(args.steps, 1), max(args.warmup, 3)
+    K, W = args.steps, max(args.warmup, 3)
     hbm_peak, peak_src = measured_peaks()
 
     # ------------------------------------------------------------------ reference arm (CPU)
@@ -486,8 +525,10 @@ def main():
             cpu_reference_run(wl, w, ids, nthreads)
         secs, npts = [], 0
         for _ in range(K):
-            sec, _, _, _, npts = cpu_reference_run(wl, w, ids, nthreads)
+            sec, xo, Po, ne, npts = cpu_reference_run(wl, w, ids, nthreads)
             secs.append(sec)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(x=xo, P=Po.reshape(-1, 30, 30), n_eff=ne))
         med = float(np.median(secs))
         val = npts * w["iters"] / med
         # the same loop on ONE scan with one thread: what a single scan (the step of the CUDA arm) gets from this CPU
@@ -577,6 +618,15 @@ def main():
     tm = eng.timer_stop()
     clocks = sampler.stop()
     barrier()
+    if args.dump_outputs and rank == 0:
+        g = (K - 1) % groups
+        eng.sync()
+        out = eng.fetch(want_world=True)
+        o0, o1 = int(wl["offs"][g * B]), int(wl["offs"][(g + 1) * B])
+        s = slice(g * B, (g + 1) * B)
+        dump_outputs(args.dump_outputs, dict(x=out["x"][s], P=out["P"][s].reshape(B, 30, 30), clk=out["clk"][s],
+                                             n_eff=out["n_eff"][s], world=out["world"][o0:o1]))
+        del out
     elapsed_ms = tm["total_ms"]
     if dist is not None:
         import torch

@@ -10,6 +10,8 @@ committed fixtures (tests/test_reference_golden.py: oracle on CPU, CUDA path und
   ref_stream_<kind>.npz one KILO::process frame (KILO.cc:356-398): ~50 buckets with the inertial (imu) or
                         kinematic-inertial (kin) queue drained in between; the cloud is stored in the order the
                         reference's own std::sort left it in
+  ref_tape/<test>.npz   the reference's answers to every call tests/test_oracle_vs_reference.py makes of it
+                        (tests/reftape.py), replayed where the reference library cannot be built
 """
 import os
 import sys
@@ -81,9 +83,16 @@ def stream(kind):
                         world=out["world"], n_eff=out["n_eff"], map1=mapcmp.digest(r.map_export()))
 
 
+def tapes():
+    import pytest
+    os.environ["LKREF_TAPE"] = "record"
+    assert pytest.main(["-q", "-p", "no:cacheprovider", os.path.join(ROOT, "tests", "test_oracle_vs_reference.py")]) == 0
+
+
 if __name__ == "__main__":
     bucket("leg_fusion")
     bucket("hilti")
     stream("imu")
     stream("kin")
+    tapes()
     print("reference-made golden fixtures written")

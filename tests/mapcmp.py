@@ -1,4 +1,6 @@
 """Structural comparison of two lk_map blobs (oracle export vs device download)."""
+import hashlib
+
 import numpy as np
 
 from legkilo_b200 import abi
@@ -102,6 +104,22 @@ def digest(blob):
     return np.concatenate(out) if out else np.zeros(0, DIGEST_DTYPE)
 
 
+def _compare_planes(dg, dig_ref, rtol, center_atol):
+    pl = (dig_ref["flags"] & 1).astype(bool)
+    np.testing.assert_allclose(dg["center"][pl], dig_ref["center"][pl], rtol=0, atol=center_atol)
+    np.testing.assert_allclose(dg["normal"][pl], dig_ref["normal"][pl], rtol=0, atol=rtol)
+    np.testing.assert_allclose(dg["d"][pl], dig_ref["d"][pl], rtol=1e-5, atol=1e-5)
+    np.testing.assert_allclose(dg["radius"][pl], dig_ref["radius"][pl], rtol=1e-6)
+    np.testing.assert_allclose(dg["var_nn"][pl], dig_ref["var_nn"][pl], rtol=rtol)
+    np.testing.assert_allclose(dg["var_cc"][pl], dig_ref["var_cc"][pl], rtol=rtol)
+
+
+def _stats(dg):
+    f = dg["flags"]
+    interior = ((f & 2) != 0) & ((f & 1) == 0) & (((f >> 16) & 0xff) != 0)
+    return dict(nodes=len(dg), planes=int((f & 1).sum()), interior=int(interior.sum()), points=int(dg["pts_count"][~interior].sum()))
+
+
 def compare_digest(dig_ref, blob, rtol=1e-6, center_atol=1e-10):
     """dig_ref: digest() of the reference's map (a committed fixture); blob: the map under test."""
     dg = digest(blob)
@@ -110,11 +128,42 @@ def compare_digest(dig_ref, blob, rtol=1e-6, center_atol=1e-10):
     np.testing.assert_array_equal(dg["flags"], dig_ref["flags"])
     np.testing.assert_array_equal(dg["pts_count"], dig_ref["pts_count"])
     np.testing.assert_array_equal(dg["new_points"], dig_ref["new_points"])
-    pl = (dig_ref["flags"] & 1).astype(bool)
-    np.testing.assert_allclose(dg["center"][pl], dig_ref["center"][pl], rtol=0, atol=center_atol)
-    np.testing.assert_allclose(dg["normal"][pl], dig_ref["normal"][pl], rtol=0, atol=rtol)
-    np.testing.assert_allclose(dg["d"][pl], dig_ref["d"][pl], rtol=1e-5, atol=1e-5)
-    np.testing.assert_allclose(dg["radius"][pl], dig_ref["radius"][pl], rtol=1e-6)
-    np.testing.assert_allclose(dg["var_nn"][pl], dig_ref["var_nn"][pl], rtol=rtol)
-    np.testing.assert_allclose(dg["var_cc"][pl], dig_ref["var_cc"][pl], rtol=rtol)
-    return dict(nodes=len(dg), planes=int(pl.sum()))
+    _compare_planes(dg, dig_ref, rtol, center_atol)
+    return _stats(dg)
+
+
+SUMMARY_PLANES = 16
+
+
+def _structure_hash(dg):
+    h = hashlib.sha256()
+    for k in ("key", "flags", "pts_count", "new_points"):
+        h.update(np.ascontiguousarray(dg[k], "<i8").tobytes())
+    return h.hexdigest()
+
+
+def summary(blob):
+    """digest() shrunk for fixtures: the node count, a hash of every node's structure (root key, flags, point counts) and
+    the digest records of a seeded sample of SUMMARY_PLANES plane nodes."""
+    dg = digest(blob)
+    planes = np.flatnonzero(dg["flags"] & 1)
+    idx = np.sort(np.random.default_rng(len(dg)).choice(planes, min(SUMMARY_PLANES, len(planes)), replace=False))
+    return dict(nodes=len(dg), structure=_structure_hash(dg), sample_idx=idx.astype(np.int32), sample=dg[idx])
+
+
+def compare_summary(summ, blob, rtol=1e-6, center_atol=1e-10):
+    """summ: summary() of the reference's map; blob: the map under test. Structure exactly, sampled planes to tolerance."""
+    dg = digest(blob)
+    assert len(dg) == summ["nodes"], (len(dg), summ["nodes"])
+    assert _structure_hash(dg) == summ["structure"], "map structure (root keys, node flags, point counts) differs from the reference's"
+    _compare_planes(dg[summ["sample_idx"]], summ["sample"], rtol, center_atol)
+    return _stats(dg)
+
+
+def compare_maps(ref, blob, rtol=1e-6, pt_atol=1e-12, var_rtol=1e-9):
+    """ref: a reference map as tests/reftape.py hands it out; blob: the map under test. Node by node and point by point
+    with compare_blobs where the reference's whole export is at hand, against its summary always."""
+    st = compare_summary(ref.summary, blob, rtol=rtol, center_atol=max(pt_atol, 1e-12))
+    if ref.blob is not None:
+        st = compare_blobs(ref.blob, blob, rtol=rtol, pt_atol=pt_atol, var_rtol=var_rtol)
+    return st
