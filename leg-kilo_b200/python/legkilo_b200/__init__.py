@@ -277,6 +277,14 @@ class Engine:
         self._chk(lib().lk_debug_residuals(self.h, _p(x), _p(P), _p(pts), n, _p(ok), _p(h), _p(z), _p(R), _p(key)))
         return dict(ok=ok, h=h, z=z, R=R, key=key)
 
+    def debug_partials(self, n_chunks: int) -> np.ndarray:
+        """Per-chunk partial rows of the last multi-kernel residual pass (lk_debug_read, what = 0): [n_chunks, 32]
+        doubles, A = sum h^T h / R upper triangle row-major (21) | b = sum h z / R (6) | sum R | count | pad. The
+        persistent per-scan kernel (fused, batch of one) keeps its partials elsewhere and leaves these alone."""
+        out = np.zeros((n_chunks, 32))
+        self._chk(lib().lk_debug_read(self.h, 0, _p(out), out.nbytes))
+        return out
+
     def update_by_points(self, x, P, h, z, R):
         """ESKF::updateByPoints (eskf.cc:91-113) from explicit rows."""
         x = np.array(x, abi.STATE_DTYPE, copy=True); P = np.array(P, np.float64, copy=True).reshape(900)
